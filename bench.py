@@ -18,6 +18,7 @@ Nested records in the same JSON line, each with its own roofline:
 
   python bench.py --gpus N --steps K --warmup W            # our CUDA path (N>1 under torchrun, weak scaling)
   python bench.py --impl reference ...                     # the reference algorithm on the host CPU cores (oracle port), same workload
+  python bench.py ... --dump-outputs DIR                   # also write what the last timed headline step computed, as DIR/*.npy
 
 One JSON line on stdout (rank 0).
 """
@@ -32,6 +33,7 @@ import sys
 import threading
 import time
 
+import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
@@ -375,9 +377,11 @@ def build_llm(env, layers):
     return model
 
 
-def run_c5(env, model, steps, warmup):
+def run_c5(env, model, steps, warmup, dump_dir=None):
     """Headline: stage-1 creation training step.  Whole fwd+bwd replayed as ONE CUDA graph (static layout: the collator's index maps are
-    built once), then — outside the graph — gradient all-reduce (N > 1), global-norm clip and fused AdamW on the flat trainable bucket."""
+    built once), then — outside the graph — gradient all-reduce (N > 1), global-norm clip and fused AdamW on the flat trainable bucket.
+    `dump_dir`: write what the last timed step hands its caller — the loss, the trainable parameters after its AdamW update and the
+    gradients it applied (flat, in `trainable` order, 2 x 17.8 MB) — as fp32 .npy files, so two builds can be compared output for output."""
     from dreamllm_b200 import ops
     from dreamllm_b200.modeling_plugins import DreamEmbedding, StableDiffusionHead, build_splice_plan
     dev, world, rank, dist = env.dev, env.world, env.rank, env.dist
@@ -489,6 +493,10 @@ def run_c5(env, model, steps, warmup):
         step_e2e()
     total = env.timed(step_dev, steps)
     total_e2e = env.timed(step_e2e, steps)
+    if dump_dir:
+        os.makedirs(dump_dir, exist_ok=True)
+        for name, t in (("c5_loss", loss_static), ("c5_trainable_params", flat_p[:n_tr]), ("c5_trainable_grads", flat_g[:n_tr])):
+            np.save(os.path.join(dump_dir, f"{name}.npy"), t.float().cpu().numpy())
     toks, pix = B * S * world, B * R * R * world
     ms, ms_e = total / steps, total_e2e / steps
     fl = c5_flops_per_gpu(B, S)
@@ -764,6 +772,8 @@ def main():
     ap.add_argument("--only", default="", help="dev only: comma list of records to run (c5,c2,c4,c3,c1)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--fast", action="store_true", help="skip the slow CPU legs (c1 in full, c2 sample)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the loss, updated trainable parameters and gradients of the last timed "
+                                                          "headline step to DIR/*.npy (fp32); inputs are seeded, identical run to run")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", 0))
 
@@ -785,8 +795,8 @@ def main():
     # order: c1 / c2 / c3 need every LLM weight trainable; c5 re-freezes the LLM, so it runs after them; c4 is independent
     for name, fn in (("c1", lambda: run_c1(env, model)),
                      ("c2", lambda: run_c2(env, model, args.steps, args.warmup, args.bs, args.seq, args.layers)),
-                     ("c3", lambda: run_c3(env, model, min(args.steps, 3), 2)),
-                     ("c5", lambda: run_c5(env, model, args.steps, args.warmup)),
+                     ("c3", lambda: run_c3(env, model, args.steps, 2)),
+                     ("c5", lambda: run_c5(env, model, args.steps, args.warmup, args.dump_outputs if rank == 0 else None)),
                      ("c4", lambda: run_c4(env))):
         if name not in only:
             continue

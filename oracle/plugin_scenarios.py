@@ -1,13 +1,14 @@
 """TEST INFRASTRUCTURE — deterministic scenarios for the plugin-level oracles (splice / conditioning gather / loss combination /
-diffusion loss), shared by
-  * tests/test_oracle_pin_model.py, tests/test_oracle_pin_sdhead.py  (oracle == LIVE reference, build container only),
-  * oracle/gen_golden_plugins.py                                    (mints tests/golden/plugins.npz from the LIVE reference),
-  * tests/test_golden_plugins.py                                    (oracle == golden, runs anywhere).
-`live_*` functions exec the reference's own methods verbatim from /root/reference (modeling_dreamllm.py:1045-1158, :1353-1509;
-modeling_plugins.py:468-577) with stand-in sub-modules; `oracle_*` functions compute the same quantities with the restatements.
-Never imported by the product."""
+diffusion loss / CFG rescale / config defaults), shared by
+  * oracle/gen_golden_plugins.py   (mints tests/golden/plugins.npz and tests/golden/reference_config.json from the LIVE reference),
+  * tests/test_golden_plugins.py, tests/test_oracle_pin_model.py, tests/test_oracle_pin_sdhead.py, tests/test_scheduler_cpu.py,
+    tests/test_hf_surface_cpu.py   (oracle / product == golden, run anywhere).
+`live_*` functions exec the reference's own methods verbatim from a reference checkout (modeling_dreamllm.py:1045-1158, :1353-1509;
+modeling_plugins.py:468-577, :658-669; configuration_dreamllm.py:64-278) with stand-in sub-modules; `oracle_*` functions compute the
+same quantities with the restatements.  Never imported by the product."""
 from __future__ import annotations
 
+import copy
 import math
 import os
 import textwrap
@@ -24,6 +25,7 @@ from . import unet_oracle as UO
 
 REF_MODEL = "/root/reference/omni/models/dreamllm/modeling_dreamllm.py"
 REF_PLUGINS = "/root/reference/omni/models/dreamllm/modeling_plugins.py"
+REF_CONFIG = os.path.join(os.path.dirname(REF_MODEL), "configuration_dreamllm.py")
 TOK = {"<im_start>": 90, "<im_patch>": 91, "<im_end>": 92, "<dream_start>": 93, "<dream_end>": 94}
 ST = {"additional_special_tokens": TOK, "<s>": 1, "</s>": 2}
 P, Q, H, V = 5, 3, 16, 96
@@ -37,7 +39,7 @@ SDHEAD_CASES = [(0.0, 0.0, None, None), (0.1, 0.0, None, None), (0.0, 0.1, None,
 
 
 def reference_available() -> bool:
-    return os.path.isfile(REF_MODEL) and os.path.isfile(REF_PLUGINS)
+    return all(os.path.isfile(f) for f in (REF_MODEL, REF_PLUGINS, REF_CONFIG))
 
 
 # ------------------------------------------------------------------------------------------------ shared inputs
@@ -81,6 +83,31 @@ def sdhead_parts():
     enc = torch.randn(3, 5, 40, generator=g)
     u_row = torch.randn(1, 5, 40, generator=g)
     return unet, proj, lat, enc, u_row
+
+
+def rescale_inputs():
+    """(cfg, text) for `rescale_noise_cfg` at guidance 7.5"""
+    g = torch.Generator().manual_seed(0)
+    text, uncond = torch.randn(3, 4, 8, 8, generator=g) * 1.3, torch.randn(3, 4, 8, 8, generator=g)
+    return uncond + 7.5 * (text - uncond), text
+
+
+class Tok:
+    """tokenizer stand-in: length + the special-token ids of TOK / ST"""
+
+    def __init__(self, n):
+        self.n = n
+        self.pad_token_id = 0
+
+    def __len__(self):
+        return self.n
+
+    def convert_tokens_to_ids(self, t):
+        table = {**TOK, "<s>": 1, "</s>": 2}
+        return [table[x] for x in t] if isinstance(t, list) else table[t]
+
+
+CONFIG_TOKENS = {"additional_special_tokens": ["<im_start>", "<dream_start>"], "bos_token": "<s>"}
 
 
 def sdhead_replay(seed, lat, noise_offset, input_perturbation, drop_prob):
@@ -239,3 +266,40 @@ def live_sdhead(noise_offset, input_perturbation, snr_gamma, drop_prob):
     torch.manual_seed(seed)
     with torch.no_grad():
         return head.forward(torch.zeros(3, 3, 64, 64), enc, u_enc)
+
+
+def live_sdhead_dummy():
+    """the reference's images=None branch (:500-509), which only feeds DDP's unused-parameter check"""
+    head, _, _, _ = live_sdhead_object(0.0, 0.0, None, None)
+    with torch.no_grad():
+        return head.forward(None, None, None, dream_embeddings=torch.randn(1, 5, 40))
+
+
+def live_rescale_noise_cfg():
+    """`_rescale_noise_cfg` (modeling_plugins.py:658-669) on `rescale_inputs()` at guidance_rescale 0.7"""
+    src = open(REF_PLUGINS).read()
+    a = src.index("    def _rescale_noise_cfg(")
+    b = src.index("    @torch.no_grad()", a)
+    ns = {"torch": torch}
+    exec(textwrap.dedent(src[a:b]), ns)
+    cfg, text = rescale_inputs()
+    return ns["_rescale_noise_cfg"](None, cfg, text, 0.7)
+
+
+def live_config():
+    """The reference's `DreamLLMConfig` (configuration_dreamllm.py:64-278) on the installed transformers: a default instance, and one
+    after `update_special_tokens2ids_dict(CONFIG_TOKENS, Tok(96))`."""
+    from transformers import PretrainedConfig
+
+    class _Log:
+        def warning(self, *a, **k):
+            pass
+        info = warning
+
+    src = open(REF_CONFIG).read().split("\n")
+    ns = dict(PretrainedConfig=PretrainedConfig, logger=_Log(), CLASS_KEY="_class_", NAME_KEY="_name_", PLUGIN_TYPE_KEY="_plugin_type_")
+    exec("from __future__ import annotations\n" + "\n".join(src[63:278]), ns)
+    ref = ns["DreamLLMConfig"]()
+    defaults = copy.deepcopy({k: getattr(ref, k) for k in ref.to_dict()})
+    ref.update_special_tokens2ids_dict(CONFIG_TOKENS, Tok(96))
+    return defaults, ref.special_tokens2ids_dict

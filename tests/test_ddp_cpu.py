@@ -28,7 +28,7 @@ class Net(nn.Module):
         return self.b(torch.tanh(self.a(x)))
 
 
-def _worker(rank, world, port, q):
+def _worker(rank, world, port, q, done):
     os.environ["MASTER_ADDR"] = "127.0.0.1"
     os.environ["MASTER_PORT"] = str(port)
     dist.init_process_group("gloo", rank=rank, world_size=world)
@@ -43,19 +43,21 @@ def _worker(rank, world, port, q):
         net(x[rank * 4:(rank + 1) * 4]).pow(2).mean().backward()
         red.finalize()
     q.put((rank, {k: v.grad.clone() for k, v in net.named_parameters()}, red.launched))
+    done.wait(240)                    # the queued tensors live in this process's shared memory until the parent has received them
     dist.destroy_process_group()
 
 
 def _run_two_ranks():
     ctx = mp.get_context("spawn")
-    q = ctx.Queue()
+    q, done = ctx.Queue(), ctx.Event()
     port = _free_port()
-    procs = [ctx.Process(target=_worker, args=(r, 2, port, q)) for r in range(2)]
+    procs = [ctx.Process(target=_worker, args=(r, 2, port, q, done)) for r in range(2)]
     for p in procs:
         p.start()
     try:
         res = [q.get(timeout=240) for _ in range(2)]
     finally:
+        done.set()
         for p in procs:
             p.join(timeout=60)
             if p.is_alive():

@@ -10,49 +10,27 @@ import torch
 from dreamllm_b200.configuration_dreamllm import ConfigAndInitKwargs, DreamLLMConfig, deep_instantiate
 from dreamllm_b200.modeling_dreamllm import DreamLLMForCausalMLM, KVCache
 from dreamllm_b200.modeling_plugins import DreamEmbedding
+from oracle.plugin_scenarios import CONFIG_TOKENS, Tok
 
-REF_CFG = "/root/reference/omni/models/dreamllm/configuration_dreamllm.py"
+REF_CFG = os.path.join(os.path.dirname(__file__), "golden", "reference_config.json")
 TINY = dict(vocab_size=96, hidden_size=128, intermediate_size=256, num_hidden_layers=2, num_attention_heads=2)
 
 
-class Tok:
-    def __init__(self, n):
-        self.n = n
-        self.pad_token_id = 0
-
-    def __len__(self):
-        return self.n
-
-    def convert_tokens_to_ids(self, t):
-        table = {"<im_start>": 90, "<im_patch>": 91, "<im_end>": 92, "<dream_start>": 93, "<dream_end>": 94, "<s>": 1, "</s>": 2}
-        return [table[x] for x in t] if isinstance(t, list) else table[t]
-
-
-@pytest.mark.skipif(not os.path.isfile(REF_CFG), reason="reference checkout not present (GPU box)")
 def test_config_defaults_equal_the_live_reference_config():
-    """exec the reference's own class (configuration_dreamllm.py:64-278) on the installed transformers and compare every default."""
-    from transformers import PretrainedConfig
-
-    class _Log:
-        def warning(self, *a, **k):
-            pass
-        info = warning
-
-    src = open(REF_CFG).read().split("\n")
-    ns = dict(PretrainedConfig=PretrainedConfig, logger=_Log(), CLASS_KEY="_class_", NAME_KEY="_name_", PLUGIN_TYPE_KEY="_plugin_type_")
-    exec("from __future__ import annotations\n" + "\n".join(src[63:278]), ns)
-    ref, ours = ns["DreamLLMConfig"](), DreamLLMConfig()
+    """Every default against the reference's own class (configuration_dreamllm.py:64-278) on the installed transformers, as
+    tests/golden/reference_config.json recorded it (`python -m oracle.gen_golden_plugins`)."""
+    with open(REF_CFG) as f:
+        gold = json.load(f)
+    ref, ours = gold["defaults"], DreamLLMConfig()
     for k, v in ours.to_dict().items():
         if k in ("model_type", "rope_scaling"):            # transformers 5 rewrites rope_scaling=None into rope_parameters
             continue
-        assert getattr(ref, k) == v, k
-    assert ref.model_type == ours.model_type == "dreamllm"
-    tok = Tok(96)
-    tokens = {"additional_special_tokens": ["<im_start>", "<dream_start>"], "bos_token": "<s>"}
-    ref.update_special_tokens2ids_dict(tokens, tok)
-    ours.update_special_tokens2ids_dict(tokens, tok)
-    assert ref.special_tokens2ids_dict == ours.special_tokens2ids_dict == {"additional_special_tokens": {"<im_start>": 90, "<dream_start>": 93},
-                                                                           "<s>": 1}
+        assert ref[k] == v, k
+    assert ref["model_type"] == ours.model_type == "dreamllm"
+    ours.update_special_tokens2ids_dict(CONFIG_TOKENS, Tok(96))
+    assert gold["special_tokens2ids_dict"] == ours.special_tokens2ids_dict == {"additional_special_tokens": {"<im_start>": 90,
+                                                                                                             "<dream_start>": 93},
+                                                                              "<s>": 1}
 
 
 def test_plugin_registration_and_instantiation():

@@ -53,23 +53,18 @@ def test_last_ddpm_step_adds_no_noise_only_at_t0():
 
 
 def test_rescale_noise_cfg_equals_live_reference():
-    """`rescale_noise_cfg` vs the reference's `_rescale_noise_cfg` exec'd verbatim (modeling_plugins.py:658-669); formula check elsewhere."""
+    """`rescale_noise_cfg` vs the reference's `_rescale_noise_cfg` (modeling_plugins.py:658-669) on the same inputs, as
+    tests/golden/plugins.npz recorded it (`python -m oracle.gen_golden_plugins`); formula check elsewhere."""
     import os
-    import textwrap
+
+    import numpy as np
 
     from dreamllm_b200.unet import rescale_noise_cfg
-    g = torch.Generator().manual_seed(0)
-    text, uncond = torch.randn(3, 4, 8, 8, generator=g) * 1.3, torch.randn(3, 4, 8, 8, generator=g)
-    cfg = uncond + 7.5 * (text - uncond)
+    from oracle.plugin_scenarios import rescale_inputs
+    cfg, text = rescale_inputs()
     got = rescale_noise_cfg(cfg, text, 0.7)
     std = lambda x: x.flatten(1).std(dim=1).view(-1, 1, 1, 1)
     torch.testing.assert_close(got, 0.7 * cfg * std(text) / std(cfg) + 0.3 * cfg, rtol=1e-5, atol=1e-6)
     assert torch.equal(rescale_noise_cfg(cfg, text, 0.0), cfg)
-    ref = "/root/reference/omni/models/dreamllm/modeling_plugins.py"
-    if os.path.isfile(ref):
-        src = open(ref).read()
-        a = src.index("    def _rescale_noise_cfg(")
-        b = src.index("    @torch.no_grad()", a)
-        ns = {"torch": torch}
-        exec(textwrap.dedent(src[a:b]), ns)
-        assert torch.equal(got, ns["_rescale_noise_cfg"](None, cfg, text, 0.7))
+    gold = np.load(os.path.join(os.path.dirname(__file__), "golden", "plugins.npz"))
+    assert torch.equal(got, torch.from_numpy(gold["rescale_noise_cfg"]))

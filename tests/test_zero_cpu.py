@@ -220,7 +220,7 @@ def test_clipping_and_state_dict_round_trip():
 
 
 # ------------------------------------------------------------------------------------------------ world_size 2 over gloo
-def _worker(rank, world, port, q, state_dtype_name, defer=False):
+def _worker(rank, world, port, q, done, state_dtype_name, defer=False):
     os.environ["MASTER_ADDR"] = "127.0.0.1"
     os.environ["MASTER_PORT"] = str(port)
     dist.init_process_group("gloo", rank=rank, world_size=world)
@@ -238,19 +238,21 @@ def _worker(rank, world, port, q, state_dtype_name, defer=False):
         norms.append(float(opt.step(defer_gather=defer)))
     opt.wait_gathers()
     q.put((rank, {k: v.detach().clone() for k, v in net.named_parameters()}, opt.launched, opt.state_bytes_per_rank(), norms))
+    done.wait(240)                    # the queued tensors live in this process's shared memory until the parent has received them
     dist.destroy_process_group()
 
 
 def _run_two(state_dtype_name, world=2, defer=False):
     ctx = mp.get_context("spawn")
-    q = ctx.Queue()
+    q, done = ctx.Queue(), ctx.Event()
     port = _free_port()
-    procs = [ctx.Process(target=_worker, args=(r, world, port, q, state_dtype_name, defer)) for r in range(world)]
+    procs = [ctx.Process(target=_worker, args=(r, world, port, q, done, state_dtype_name, defer)) for r in range(world)]
     for p in procs:
         p.start()
     try:
         res = [q.get(timeout=240) for _ in range(world)]
     finally:
+        done.set()
         for p in procs:
             p.join(timeout=60)
             if p.is_alive():
@@ -436,7 +438,7 @@ def _branch_net():
     return BranchNet().to(BF)
 
 
-def _uneven_worker(rank, world, port, q, kind):
+def _uneven_worker(rank, world, port, q, done, kind):
     os.environ["MASTER_ADDR"] = "127.0.0.1"
     os.environ["MASTER_PORT"] = str(port)
     dist.init_process_group("gloo", rank=rank, world_size=world)
@@ -458,19 +460,21 @@ def _uneven_worker(rank, world, port, q, kind):
             net(x[rank * 4:(rank + 1) * 4], use_proj=(rank == 0)).float().pow(2).mean().backward()
             red.finalize()
         q.put((rank, {k: v.grad.detach().clone() for k, v in net.named_parameters()}))
+    done.wait(240)                    # see _worker
     dist.destroy_process_group()
 
 
 def _run_uneven(kind):
     ctx = mp.get_context("spawn")
-    q = ctx.Queue()
+    q, done = ctx.Queue(), ctx.Event()
     port = _free_port()
-    procs = [ctx.Process(target=_uneven_worker, args=(r, 2, port, q, kind)) for r in range(2)]
+    procs = [ctx.Process(target=_uneven_worker, args=(r, 2, port, q, done, kind)) for r in range(2)]
     for p in procs:
         p.start()
     try:
         res = [q.get(timeout=240) for _ in range(2)]
     finally:
+        done.set()
         for p in procs:
             p.join(timeout=60)
             if p.is_alive():
