@@ -626,11 +626,15 @@ class StableDiffusionHead(MultimodalHead):
                  cross_attention_kwargs=None, guidance_rescale: float = 0.0, scheduler: str = "ddpm", use_cuda_graph: bool = True):
         """reference :672-850.  `scheduler="ddpm"` is what the reference runs (its training DDPMScheduler, :379/:833);
         `"ddim"` (eta 0) is BASELINE.json's C4 sampler."""
-        from .unet import DenoiseLoop
+        from .unet import DenoiseLoop, check_planes
         height = height or self.resolution
         width = width or self.resolution
         if height % 8 or width % 8:
             raise ValueError(f"`height` and `width` have to be divisible by 8 but are {height} and {width}.")
+        # stricter than the reference: every UNet / VAE plane must tile the implicit-GEMM conv (DESIGN.md, divergences)
+        check_planes(height // 8, width // 8, len(self.unet.cfg["block_out_channels"]), f"UNet latents of a {height}x{width} image")
+        if output_type != "latent":
+            check_planes(height, width, len(self.vae_decoder.cfg["block_out_channels"]), f"VAE decoder planes of a {height}x{width} image")
         assert prompt_embeds is not None, "`prompt_embeds` must be provided by LLM."
         n_img = int(num_images_per_prompt or 1)
         if n_img > 1:                                           # (:760-772) each prompt's embeddings repeated per requested image

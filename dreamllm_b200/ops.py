@@ -405,6 +405,15 @@ def attn_fwd_cross(q, k, v, scale=None):
     return out
 
 
+def conv3x3_plane_supported(H: int, W: int) -> bool:
+    """The planes `dllm_conv3x3_nhwc` accepts: a 128-pixel tile is Wb x Hb x Nb pixels, so W must divide 128 or be a multiple of it,
+    and H must be a multiple of Hb = 128 / W (or divide it, when one tile spans several whole images)."""
+    if H <= 0 or W <= 0 or (W % 128 if W > 128 else 128 % W):
+        return False
+    hb = 1 if W >= 128 else 128 // W
+    return (hb % H == 0) if hb > H else (H % hb == 0)
+
+
 def conv3x3(x_nhwc, w_k, bias=None, rowbias=None, residual=None):
     """x [N,H,W,Cin] bf16 contiguous; w_k [Cout, 9*Cin] ((r,s,c)-major); returns [N,H,W,Cout]."""
     _chk_cuda(x_nhwc, w_k, bias, rowbias, residual)

@@ -487,6 +487,21 @@ class UNet2DConditionModel(nn.Module):
         return self.forward_nhwc(sample.float().contiguous(), temb_sin, self.precompute_cross_kv(encoder_hidden_states), B)
 
 
+# ------------------------------------------------------------------------------------------------ supported image sizes
+def check_planes(h: int, w: int, levels: int, what: str) -> None:
+    """Raise ValueError unless every plane h / 2^i x w / 2^i (i < levels) of a UNet or VAE runs on the implicit-GEMM conv.
+
+    The reference accepts any size divisible by 8; here every 3x3 conv is a tcgen05 implicit GEMM over 128-pixel tiles, so each plane's
+    width must divide 128 or be a multiple of it and its height must fill whole tiles (`ops.conv3x3_plane_supported`).  Checked before
+    anything is launched, so an unsupported size fails here and not inside a captured CUDA graph."""
+    for i in range(levels):
+        f = 1 << i
+        if h % f or w % f or not ops.conv3x3_plane_supported(h // f, w // f):
+            raise ValueError(f"{what} are not supported: the level-{i} plane is {h / f:g}x{w / f:g}, and every plane's "
+                             f"width must divide 128 or be a multiple of 128, and its height a multiple of 128 / width (or divide it). "
+                             f"Image sides of 256, 512 and 1024 satisfy this.")
+
+
 # ------------------------------------------------------------------------------------------------ sampler
 def scheduler_tables(num_inference_steps, kind="ddim", num_train=1000, beta_start=0.00085, beta_end=0.012, steps_offset=1):
     """SD-2.1-base scheduler_config (SURVEY Appendix A.2): scaled_linear betas, leading spacing, steps_offset 1, epsilon prediction.
@@ -538,6 +553,7 @@ class DenoiseLoop:
                  whole_loop_graph: bool = True):
         """cond: [B, Q, ctx] projected prompt embeddings, or [2B, Q, ctx] = cat([negative, positive]) when guidance_scale > 1
         (reference order, modeling_plugins.py:774-784)."""
+        check_planes(height // 8, width // 8, len(unet.cfg["block_out_channels"]), f"UNet latents of a {height}x{width} image")
         self.unet = unet
         dev = cond.device
         self.use_cfg = guidance_scale > 1.0

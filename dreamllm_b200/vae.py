@@ -13,6 +13,7 @@ import torch.nn as nn
 
 from . import ops
 from .modeling_dreamllm import _fuse_rows
+from .unet import check_planes
 
 BF16 = torch.bfloat16
 SDVAE = dict(in_channels=3, latent_channels=4, block_out_channels=(128, 256, 512, 512), layers_per_block=2, norm_num_groups=32,
@@ -120,6 +121,7 @@ class AutoencoderKLEncoder(nn.Module):
             raise RuntimeError("dreamllm_b200 VAE encoder requires CUDA tensors; there is no CPU fallback")
         e = self.encoder
         B, _, H, W = images.shape
+        check_planes(H, W, len(self.cfg["block_out_channels"]), f"VAE encoder planes of a {H}x{W} image")
         x = ops.conv_in(images.float().contiguous(), e.conv_in.weight, e.conv_in.bias, B)
         for b in e.down_blocks:
             for r in b.resnets:
@@ -188,6 +190,9 @@ class AutoencoderKLDecoder(AutoencoderKLEncoder):
             raise RuntimeError("dreamllm_b200 VAE decoder requires CUDA tensors; there is no CPU fallback")
         d = self.decoder
         L = self.cfg["latent_channels"]
+        nlev = len(self.cfg["block_out_channels"])
+        check_planes(latents.shape[2] << (nlev - 1), latents.shape[3] << (nlev - 1), nlev,
+                     f"VAE decoder planes of {tuple(latents.shape[2:])} latents")
         z = latents.float() / self.cfg["scaling_factor"]
         B = z.shape[0]
         # post_quant_conv (1x1, 4 -> 4) folded into conv_in's input: tiny, done as a per-pixel 4x4 matmul on the fp32 latents
